@@ -6,7 +6,9 @@ One "step" = one pass of the hot path over one batch of synthetic input:
     query: M UCB candidates: K*, L^-1 K*, mu, sigma^2, UCB, argmax (gp.hpp:159-167, acqui/ucb.hpp:83-90)
 at N = 16384, D = 6, SquaredExpARD, fp64, M = 10000 (SURVEY.md §8d (i)).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload ...]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload ...] [--dump-outputs DIR]
+
+It runs from the tree as __graft_entry__.build() left it and writes nothing there (the tree may be read-only).
 
 `value`   : steps/s with inputs already resident in HBM (device-pointer ABI), CUDA events on the library's stream.
 `e2e`     : the same step through the public host API (limbo_b200.model.GP.compute + acqui.UCB.argmax_batch /
@@ -418,6 +420,27 @@ def roofline_table(prof: dict, steps: int, t_ms: float, n: int, d: int, m_local:
     return rows
 
 
+DUMP_SEED, DUMP_L_ROWS = 2024, 256
+
+
+def dump_outputs(out_dir: str, lib, h, n: int, best: tuple[float, int]) -> None:
+    """--dump-outputs: what the last timed step hands its caller, as float64 .npy files, so that two builds can be compared
+    output for output: the UCB argmax (value, global index), alpha (N) and a fixed, seeded sample of DUMP_L_ROWS rows of the
+    Cholesky factor L (the whole factor is 2.1 GB at N=16384; the sample is 32 MB)."""
+    from limbo_b200 import _lib
+    L = np.empty((n, n), order="F")
+    _lib.check(lib.lb_get(h, _lib.GET_L, L.ctypes.data), "lb_get L")
+    alpha = np.empty(n)
+    _lib.check(lib.lb_get(h, _lib.GET_ALPHA, alpha.ctypes.data), "lb_get alpha")
+    rows = np.sort(np.random.default_rng(DUMP_SEED).choice(n, min(n, DUMP_L_ROWS), replace=False))
+    out = {"ucb_best_value": np.array([best[0]]), "ucb_best_index": np.array([best[1]], dtype=np.float64), "alpha": alpha,
+           "L_rows": np.ascontiguousarray(L[rows]), "L_row_index": rows.astype(np.float64)}
+    del L
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def run_config4(args, torch, dist, dev, rank, world, lib, precision: str = "tf32", m_total: int = 1_000_000, steps: int = 2) -> dict | None:
     """BASELINE.json config 4: N=16384, D=12, reduced-precision scoring, 1M EI candidates sharded over the ranks, one
     all_gather for the argmax.  The timed step includes the fp64 fit, the inversion of the factor and its cast (replicated on
@@ -615,11 +638,6 @@ def run_ours(args) -> None:
     dev = torch.device("cuda", local_rank)
     if world > 1:
         dist.init_process_group("nccl", device_id=dev)
-    import __graft_entry__ as ge
-    if rank == 0:
-        ge.build()
-    if world > 1:
-        dist.barrier()
     from limbo_b200 import _lib, acqui, kernel, mean, model, synth
     from limbo_b200 import dist as lbdist
 
@@ -731,6 +749,13 @@ def run_ours(args) -> None:
     t_ms = float(tt.item())
     ms_per_step = t_ms / steps
     value = 1.0 / (ms_per_step * 1e-3)  # global jobs per second (one job = fit + all M candidates), whatever the GPU count
+    if args.dump_outputs and rank == 0:
+        if world > 1:
+            recs = torch.stack(gather_buf).cpu().numpy()
+            best = lbdist.reduce_records(recs[:, 0], recs[:, 1].astype(np.int64))
+        else:
+            best = (float(dBest.item()), int(dIdx.item()))
+        dump_outputs(args.dump_outputs, lib, h, n, best)
 
     # ---------------- end-to-end leg through the public host API ----------------
     gp2 = model.GP(d, 1, kernel=kcls, mean=mean.Data, device=local_rank)
@@ -902,11 +927,6 @@ def run_config4_workload(args) -> None:
     dev = torch.device("cuda", lr)
     if world > 1:
         dist.init_process_group("nccl", device_id=dev)
-    import __graft_entry__ as ge
-    if rank == 0:
-        ge.build()
-    if world > 1:
-        dist.barrier()
     from limbo_b200 import _lib
     lib = _lib.load()
     prof_api(lib)
@@ -941,7 +961,10 @@ def main() -> None:
                     help="N > 1, config 4: every rank inverts the whole factor (round-1 scheme) instead of its column tiles + one all_gather")
     ap.add_argument("--workload", default="n16384_se_ard", choices=sorted(WORKLOADS) + ["config4"])
     ap.add_argument("--precision", default="tf32", choices=["tf32", "fp16"], help="--workload config4 only")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last step computed to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl == "reference" or args.workload == "config4"):
+        ap.error("--dump-outputs applies to the fit + UCB workloads of --impl ours")
     if args.workload == "config4":
         if args.impl == "reference":
             print(json.dumps({"impl": "reference", "unavailable": "config 4 is a reduced-precision GPU workload; the reference arm is defined for the headline workload"}))

@@ -1,43 +1,30 @@
-"""Pins the oracle restatement against the reference ITSELF where it can run: the reference's
-own headers compiled against the Eigen/Boost stand-in (oracle/ref_shim -> oracle/_ref).  Skipped
-where neither /root/reference nor a prebuilt oracle/_ref/libref_gp.so exists."""
+"""Pins the oracle restatement against the reference ITSELF: tests/golden/restatement/ holds what the reference's own
+headers, compiled against the Eigen/Boost stand-in (oracle/ref_shim), computed on these inputs
+(tests/golden/make_golden_restatement.py).  K and L are compared on a seeded sample of rows."""
+import os
+
 import numpy as np
 import pytest
 
-from limbo_b200 import synth
+GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "restatement")
 
 
-@pytest.fixture(scope="module")
-def ref_mod():
-    from oracle import ref
-    if not ref.available():
-        pytest.skip("reference sources not mounted and no prebuilt oracle/_ref")
-    try:
-        ref.build()
-        ref.load()
-    except Exception as e:  # noqa: BLE001
-        pytest.skip(f"reference shim build unavailable: {e}")
-    return ref
+def _gold(name):
+    return np.load(os.path.join(GOLD, name + ".npz"))
 
 
 @pytest.mark.parametrize("kid", [0, 1, 2, 3])
 @pytest.mark.parametrize("N,D,P", [(5, 1, 1), (33, 3, 2), (120, 6, 1)])
-def test_restatement_equals_reference(ref_mod, oracle_mod, kid, N, D, P):
+def test_restatement_equals_reference(oracle_mod, kid, N, D, P):
     O = oracle_mod
-    rng = np.random.default_rng(100 * kid + N)
-    nh = D + 1 if kid == 0 else 2
-    hp = rng.uniform(-0.7, 0.7, nh)
-    X = synth.points(77 + N, N, D)
-    y = synth.targets(X)
-    Y = np.stack([y * (p + 1) - 0.3 * p for p in range(P)], axis=1)
-    Xq = synth.points(78, 25, D)
-    r = ref_mod.run(kid, X, Y, 0.015, hp=hp, Xq=Xq)
+    r = _gold(f"k{kid}_n{N}_d{D}_p{P}")
+    X, Y, Xq, rows = r["X"], r["Y"], r["Xq"], r["rows"]
     og = O.OracleGP()
     og.set_data(X, Y - Y.mean(axis=0))
-    og.set_kernel(kid, hp, 0.015)
+    og.set_kernel(kid, r["hp"], float(r["noise"]))
     assert og.fit() == -1
-    assert np.abs(og.get(0) - r["K"]).max() <= 1e-15
-    assert np.abs(og.get(1) - r["L"]).max() <= 1e-12
+    assert np.abs(og.get(0)[rows] - r["K_rows"]).max() <= 1e-15
+    assert np.abs(og.get(1)[rows] - r["L_rows"]).max() <= 1e-12
     assert np.abs(og.get(2) - r["alpha"]).max() <= 1e-11 * np.abs(r["alpha"]).max()
     mu, s2 = og.query(Xq)
     assert np.abs(mu + Y.mean(axis=0) - r["mu"]).max() <= 1e-12
@@ -46,30 +33,28 @@ def test_restatement_equals_reference(ref_mod, oracle_mod, kid, N, D, P):
     assert np.abs(og.grad() - r["grad"]).max() <= 1e-10 * max(1.0, np.abs(r["grad"]).max())
 
 
-def test_rprop_trajectory_equals_reference(ref_mod, oracle_mod):
+def test_rprop_trajectory_equals_reference(oracle_mod):
     """KernelLFOpt<Rprop> in the reference vs the restated Rprop on the restated objective."""
     O = oracle_mod
-    X = synth.points(5, 50, 2)
-    y = synth.targets(X)
-    r = ref_mod.run(0, X, y, 0.01, rprop_iters=10)
+    r = _gold("rprop_n50_d2")
+    X, Y = r["X"], r["Y"]
     og = O.OracleGP()
-    og.set_data(X, (y - y.mean())[:, None])
-    og.set_kernel(0, np.zeros(3), 0.01)
+    og.set_data(X, Y - Y.mean())
+    og.set_kernel(0, np.zeros(3), float(r["noise"]))
     og.fit()
-    best, ne = og.rprop_lml(np.zeros(3), 10)
+    best, ne = og.rprop_lml(np.zeros(3), int(r["rprop_iters"]))
     assert ne == 10 and np.abs(best - r["hp"]).max() <= 1e-12
 
 
-def test_incremental_equals_reference(ref_mod, oracle_mod):
+def test_incremental_equals_reference(oracle_mod):
     O = oracle_mod
-    X = synth.points(6, 40, 2)
-    y = synth.targets(X)[:, None]
-    r = ref_mod.run(1, X, y, 0.01, n0=25)
+    r = _gold("incremental_n40_d2")
+    X, y, n0, rows = r["X"], r["Y"], int(r["n0"]), r["rows"]
     og = O.OracleGP()
-    og.set_data(X[:25], y[:25] - y[:25].mean())
-    og.set_kernel(1, np.zeros(2), 0.01)
+    og.set_data(X[:n0], y[:n0] - y[:n0].mean())
+    og.set_kernel(1, np.zeros(2), float(r["noise"]))
     og.fit()
-    for i in range(25, 40):
+    for i in range(n0, X.shape[0]):
         og.append(X[i], y[: i + 1] - y[: i + 1].mean())
-    assert np.abs(og.get(1) - r["L"]).max() <= 1e-12
+    assert np.abs(og.get(1)[rows] - r["L_rows"]).max() <= 1e-12
     assert np.abs(og.get(2) - r["alpha"]).max() <= 1e-11 * np.abs(r["alpha"]).max()
