@@ -146,6 +146,17 @@ int lb_kernel_grad_log_loo_cv(lb_gp* h, int optimize_noise, double* grad);
  * caller contracts it with its mean functor's gradient (mean/mean.hpp:72-76), which is host code. */
 int lb_kinv_obs_mean(lb_gp* h, double* out_colmajor);
 
+/* model::SparsifiedGP::_sparsify (model/sparsified_gp.hpp:126-183): greedy density-based selection of max_points of the N
+ * samples (row-major N x D).  The density of a point is the sum of its D smallest Euclidean distances to the other
+ * remaining points, added in ascending order; the point of smallest density is removed, the lowest index on a tie (the
+ * reference's sequential scan), until max_points remain.  keep_idx receives the min(N, max_points) kept indices in
+ * ascending order; removed_idx / removed_density (optional, NULL) the N - max_points removals in order and the density
+ * at which each point went.  N <= max_points returns the identity and launches nothing.  LB_ERR_ARG for N < 1, D < 1,
+ * D > 64 or max_points < D (the reference's partial_sort would then read past its row).  The handle's data, kernel,
+ * factor and alpha are left as they are; its workspace is used, so the call needs exclusive access to the handle. */
+int lb_sparsify(lb_gp* h, int64_t N, int D, const double* X_rowmajor, int64_t max_points,
+    int64_t* keep_idx, int64_t* removed_idx, double* removed_density);
+
 /* accessors matrixL(), alpha(), ... (gp.hpp:411-436): dst is column-major,
  * N x N (K, L, KINV) or N x P (ALPHA). */
 int lb_get(lb_gp* h, int what, double* dst_colmajor);

@@ -21,7 +21,7 @@ DECLARED_SYMBOLS = [
     "lb_create", "lb_destroy", "lb_clone", "lb_set_stream", "lb_sync", "lb_launch_count", "lb_set_data",
     "lb_set_data_dev", "lb_set_kernel", "lb_fit", "lb_load_factor", "lb_refit_alpha", "lb_append", "lb_query", "lb_query_dev",
     "lb_acq_argmax", "lb_acq_argmax_dev", "lb_log_lik", "lb_kernel_grad_log_lik", "lb_compute_inv_kernel", "lb_log_loo_cv",
-    "lb_kernel_grad_log_loo_cv", "lb_kinv_obs_mean", "lb_get",
+    "lb_kernel_grad_log_loo_cv", "lb_kinv_obs_mean", "lb_sparsify", "lb_get",
     "lb_nb_samples", "lb_strerror", "lb_last_cuda_error",
 ]
 
@@ -86,6 +86,7 @@ def load() -> C.CDLL:
         "lb_log_loo_cv": ([p, dp], i32),
         "lb_kernel_grad_log_loo_cv": ([p, i32, dp], i32),
         "lb_kinv_obs_mean": ([p, dp], i32),
+        "lb_sparsify": ([p, i64, i32, dp, i64, dp, dp, dp], i32),
         "lb_get": ([p, i32, dp], i32),
         "lb_nb_samples": ([p], i64),
         "lb_strerror": ([i32], C.c_char_p),

@@ -16,7 +16,9 @@ from .gp import GP
 
 class MultiGP:
     def __init__(self, dim_in: int = -1, dim_out: int = -1, params=None, kernel=_kernel.MaternFiveHalves, mean=_mean.Data,
-                 hp_opt=None, device: int = 0, devices=None):
+                 hp_opt=None, device: int = 0, devices=None, gp=GP):
+        # gp: the per-output model class, the reference's template-template argument (multi_gp.hpp:59), e.g. SparsifiedGP
+        self._gp_cls = gp
         self._params = params
         self._kernel_cls, self._mean_cls = kernel, mean
         self._dim_in, self._dim_out = dim_in, dim_out
@@ -33,7 +35,7 @@ class MultiGP:
             self._gp_models = [self._make_gp(i) for i in range(dim_out)]
 
     def _make_gp(self, i: int) -> GP:
-        return GP(self._dim_in if self._dim_in > 0 else -1, 1, params=self._params, kernel=self._kernel_cls, mean=_mean.NullFunction,
+        return self._gp_cls(self._dim_in if self._dim_in > 0 else -1, 1, params=self._params, kernel=self._kernel_cls, mean=_mean.NullFunction,
                   device=self._devices[i % len(self._devices)])
 
     def _update_mean_observation(self) -> None:

@@ -45,6 +45,9 @@ class defaults:
         repeats = 10
         epsilon = 1e-2
 
+    class model_sparse_gp:  # model/sparsified_gp.hpp:56-59
+        max_points = 200
+
     class bayes_opt_boptimizer:  # bayes_opt/boptimizer.hpp:68-72
         hp_period = -1
 
