@@ -64,6 +64,7 @@ def load() -> C.CDLL:
         "lb_debug_pool_hits": ([], C.c_longlong),
         "lb_pool_trim": ([], i32),
         "lb_debug_set_query_panel_min": ([C.c_longlong], i32),
+        "lb_debug_set_query_int8": ([C.c_int, C.c_longlong], i32),
         "lb_set_data": ([p, i64, i32, i32, dp, dp], i32),
         "lb_set_data_dev": ([p, i64, i32, i32, dp, dp], i32),
         "lb_set_kernel": ([p, i32, dp, i32, dbl], i32),

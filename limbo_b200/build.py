@@ -15,7 +15,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIBDIR = os.path.join(HERE, "lib")
 LIB = os.path.join(LIBDIR, "liblimbo_b200.so")
-SOURCES = ["abi.cu", "pool.cu", "kbuild.cu", "potrf.cu", "trsv.cu", "query.cu", "lml.cu", "loo.cu", "tf32_query.cu", "sparsify.cu"]
+SOURCES = ["abi.cu", "pool.cu", "kbuild.cu", "potrf.cu", "trsv.cu", "query.cu", "query_i8.cu", "lml.cu", "loo.cu", "tf32_query.cu", "sparsify.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
     "--extended-lambda", "-Xcompiler", "-fPIC", "-diag-suppress", "177",

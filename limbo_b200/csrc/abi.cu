@@ -29,7 +29,7 @@ int lb_dinv_pack_impl(lb_gp* h, const double* dV, int rank, int G, double absmax
 int lb_dinv_adopt_impl(lb_gp* h, int G, const void* dAll, double absmax_all);
 int lb_launch_query_point(const lb_gp* h, cudaStream_t st, const double* x_host, double* dQs, double* dVscratch, double* dOutMapped,
     long long* launches);
-int lb_launch_query_panel(lb_gp* h, cudaStream_t st, int64_t M, const double* dQs, int64_t Mp, double* dWork, double* dMu, double* dS2,
+int lb_launch_query_panel(lb_gp* h, cudaStream_t st, int64_t M, const double* dQs, int64_t Mp, double* dWork, double* dMu, double* dS2, int* dErr,
     long long* launches);
 size_t lb_query_fused_scratch_doubles(const lb_gp* h, int grid);
 int lb_launch_query_fused(const lb_gp* h, cudaStream_t st, int64_t M, const double* dQs, int64_t Mp, double* dVscratch,
@@ -262,8 +262,10 @@ void free_ws(QueryWs& w)
 
 void free_model(lb_gp* h)
 {
-    void* all[] = {h->dX, h->dXs, h->dY, h->dL, h->dInvD, h->dAlpha, h->dLinv, h->dKinv, h->dFlags, h->dLinv32, h->dWork, h->dLinvW, h->dTrsvX};
+    void* all[] = {h->dX, h->dXs, h->dY, h->dL, h->dInvD, h->dAlpha, h->dLinv, h->dKinv, h->dFlags, h->dLinv32, h->dWork, h->dLinvW, h->dTrsvX,
+        h->dLdig};
     h->dTrsvX = nullptr; h->trsvx_np = 0;
+    h->dLdig = nullptr; h->ldig_np = 0; h->ldig_valid = false;
     for (void* p : all) lb_pool_free(p); // shared buffers (lb_clone) only lose this handle's reference
     h->dWork = nullptr; h->work_np = 0; h->dLinvW = nullptr; h->linvw_np = 0;
     h->dLinv32 = nullptr; h->linv32_valid = false; h->linv32_rows = 0;
@@ -462,7 +464,7 @@ static int set_data_common(lb_gp* h, int64_t N, int D, int P, const double* X, c
     h->N = N; h->D = D; h->P = P;
     h->kp.Draw = D;
     h->kp.D = D + h->kp.klam;
-    h->fitted = false; h->linv_valid = false; h->linv_levels = 0; h->kinv_valid = false; h->linv32_valid = false;
+    h->fitted = false; h->linv_valid = false; h->linv_levels = 0; h->ldig_valid = false; h->kinv_valid = false; h->linv32_valid = false;
     const double* dXr = X;
     const double* dYr = Y;
     if (!dev && N > 0) {
@@ -497,7 +499,7 @@ int lb_dchol_set_points(lb_gp* h, int64_t N, int D, const double* X)
     h->N = N; h->D = D; h->P = 0;
     h->kp.Draw = D;
     h->kp.D = D + h->kp.klam;
-    h->fitted = false; h->linv_valid = false; h->linv_levels = 0; h->kinv_valid = false; h->linv32_valid = false;
+    h->fitted = false; h->linv_valid = false; h->linv_levels = 0; h->ldig_valid = false; h->kinv_valid = false; h->linv32_valid = false;
     int rc = lb_ensure_scratch(h, sizeof(double) * (size_t)N * D);
     if (rc) return rc;
     LB_CUDA(cudaMemcpyAsync(h->dScratch, X, sizeof(double) * N * D, cudaMemcpyHostToDevice, h->stream));
@@ -574,7 +576,7 @@ int lb_set_kernel(lb_gp* h, int kernel_id, const double* p, int n_hparams, doubl
         && old.sf2 == kp.sf2 && old.l == kp.l && old.noise == kp.noise && old.c1 == kp.c1 && old.c2 == kp.c2;
     if (same && kernel_id == LB_K_SE_ARD)
         for (int d = 0; d < h->D; ++d) same = same && (old.inv_ell[d] == kp.inv_ell[d]);
-    if (!same) { h->fitted = false; h->linv_valid = false; h->linv_levels = 0; h->kinv_valid = false; h->linv32_valid = false; }
+    if (!same) { h->fitted = false; h->linv_valid = false; h->linv_levels = 0; h->ldig_valid = false; h->kinv_valid = false; h->linv32_valid = false; }
     return LB_OK;
 }
 
@@ -589,7 +591,7 @@ int lb_fit(lb_gp* h)
     if ((rc = lb_launch_scale_x(h))) return rc;
     if ((rc = lb_launch_kbuild(h, h->dL))) return rc;
     if ((rc = lb_launch_potrf(h))) return rc;
-    h->fitted = true; h->linv_valid = false; h->linv_levels = 0; h->kinv_valid = false; h->linv32_valid = false;
+    h->fitted = true; h->linv_valid = false; h->linv_levels = 0; h->ldig_valid = false; h->kinv_valid = false; h->linv32_valid = false;
     if ((rc = lb_launch_solve_alpha(h))) return rc;
     return check_info(h);
 }
@@ -604,7 +606,7 @@ int lb_fit_async(lb_gp* h) // same as lb_fit without the final host sync / info 
     if ((rc = lb_launch_scale_x(h))) return rc;
     if ((rc = lb_launch_kbuild(h, h->dL))) return rc;
     if ((rc = lb_launch_potrf(h))) return rc;
-    h->fitted = true; h->linv_valid = false; h->linv_levels = 0; h->kinv_valid = false; h->linv32_valid = false;
+    h->fitted = true; h->linv_valid = false; h->linv_levels = 0; h->ldig_valid = false; h->kinv_valid = false; h->linv32_valid = false;
     return lb_launch_solve_alpha(h);
 }
 
@@ -672,7 +674,7 @@ int lb_load_factor(lb_gp* h, const double* L_colmajor, const double* alpha_colma
     h->launches++;
     for (int k = 0; k < T; ++k)
         if ((rc = lb_launch_potf2_block(h, k, 0))) return rc;
-    h->fitted = true; h->linv_valid = false; h->linv_levels = 0; h->kinv_valid = false; h->linv32_valid = false;
+    h->fitted = true; h->linv_valid = false; h->linv_levels = 0; h->ldig_valid = false; h->kinv_valid = false; h->linv32_valid = false;
     return check_info(h);
 }
 
@@ -761,7 +763,7 @@ int lb_append(lb_gp* h, const double* x, const double* Yall)
     append_row_kernel<<<1, 256, 0, h->stream>>>(h->dL, Np, n, dk, knn, h->dInfo);
     h->launches++;
     if ((rc = lb_launch_potf2_block(h, (int)(n / LB_TILE), 0))) return rc;
-    h->linv_valid = false; h->linv_levels = 0; h->kinv_valid = false; h->linv32_valid = false;
+    h->linv_valid = false; h->linv_levels = 0; h->ldig_valid = false; h->kinv_valid = false; h->linv32_valid = false;
     if ((rc = lb_launch_solve_alpha(h))) return rc;
     return check_info(h);
 }
@@ -879,13 +881,24 @@ static int query_common(const lb_gp* hc, int64_t M, const double* Xq, bool xq_de
             const int64_t Mc = std::min(Mp, maxcols);
             if ((rc = ensure(h, &w.dQs, &w.qs_bytes, sizeof(double) * De * Mc))) return rc;
             if ((rc = ensure(h, &w.dV, &w.v_bytes, sizeof(double) * lb_query_panel_scratch_doubles(h, Mc)))) return rc;
+            const bool i8 = lb_query_int8_mode() != 0; // the int8 update's mbarrier waits are bounded and raise w.dErr
+            if (i8) {
+                if (!w.dErr) LB_ALLOC(h, w.dErr, sizeof(int));
+                LB_CUDA(cudaMemsetAsync(w.dErr, 0, sizeof(int), st));
+            }
             for (int64_t m0 = 0; m0 < M; m0 += Mc) {
                 const int64_t mc = std::min(Mc, M - m0);
                 const int64_t mcp = (mc + LB_TILE - 1) / LB_TILE * LB_TILE;
                 dim3 g1((unsigned)((mcp + 255) / 256), (unsigned)De);
                 pack_soa_kernel<<<g1, 256, 0, st>>>(dQraw + m0 * D, mc, D, w.dQs, mcp, h->kp, 1);
                 h->launches++;
-                if ((rc = lb_launch_query_panel(h, st, mc, w.dQs, mcp, w.dV, w.dMu + m0 * P, w.dS2 + m0, &h->launches))) return rc;
+                if ((rc = lb_launch_query_panel(h, st, mc, w.dQs, mcp, w.dV, w.dMu + m0 * P, w.dS2 + m0, w.dErr, &h->launches))) return rc;
+            }
+            if (i8 && !out_dev) {
+                int herr = 0;
+                LB_CUDA(cudaMemcpyAsync(&herr, w.dErr, sizeof(int), cudaMemcpyDeviceToHost, st));
+                LB_CUDA(cudaStreamSynchronize(st));
+                if (herr) return LB_ERR_TIMEOUT;
             }
         }
         else if (lb_query_fused_supported(h) && !h->force_unfused) {
@@ -1171,6 +1184,10 @@ int lb_clone(const lb_gp* src, lb_gp** out)
             h->dL = share(src->dL);
             h->dInvD = share(src->dInvD);
             h->fitted = true;
+            if (src->ldig_valid) { // digit planes of the shared factor (the panel query's int8 update)
+                lb_pool_retain(src->dLdig);
+                h->dLdig = src->dLdig; h->ldig_np = src->ldig_np; h->ldig_valid = true;
+            }
         }
         if (src->dFlags && lb_dalloc(h, &h->dFlags, sizeof(int) * (src->Np / LB_TILE + 8))) { lb_destroy(h); return LB_ERR_ALLOC; }
     }
@@ -1241,7 +1258,7 @@ int lb_dchol_adopt_begin(lb_gp* h, int64_t Nd)
     if ((rc = ensure_fit_buffers(h))) return rc;
     if ((rc = lb_launch_scale_x(h))) return rc;
     LB_CUDA(cudaMemsetAsync(h->dInfo, 0, 2 * sizeof(int), h->stream));
-    h->fitted = false; h->linv_valid = false; h->linv_levels = 0; h->kinv_valid = false; h->linv32_valid = false;
+    h->fitted = false; h->linv_valid = false; h->linv_levels = 0; h->ldig_valid = false; h->kinv_valid = false; h->linv32_valid = false;
     return LB_OK;
 }
 // one received (or own) panel message into the handle's L / invD, on `stream` (cudaStream_t as void*; NULL = the handle's)
@@ -1263,7 +1280,7 @@ int lb_dchol_adopt_end(lb_gp* h, int info)
     if (!h) return LB_ERR_ARG;
     LB_DEVICE(h);
     if (info > 0) return info;
-    h->fitted = true; h->linv_valid = false; h->linv_levels = 0; h->kinv_valid = false; h->linv32_valid = false;
+    h->fitted = true; h->linv_valid = false; h->linv_levels = 0; h->ldig_valid = false; h->kinv_valid = false; h->linv32_valid = false;
     int rc = lb_launch_solve_alpha(h);
     if (rc) return rc;
     return check_info(h);

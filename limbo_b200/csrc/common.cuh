@@ -309,6 +309,7 @@ struct lb_gp {
     double* dAlpha = nullptr; // Np x P
     double* dLinv = nullptr; // Np x Np (lazy: L^-1)
     double* dKinv = nullptr; // Np x Np (lazy: K^-1, lower valid + mirrored)
+    int8_t* dLdig = nullptr; int64_t ldig_np = 0; bool ldig_valid = false; // panel query: int8 digit planes of L (query_i8.cu)
     float* dLinv32 = nullptr; int64_t linv32_rows = 0; bool linv32_valid = false; double linv32_scale = 1.0; // reduced-precision path: row-major fp32 / fp16 L^-1
     int* dInfo = nullptr;    // [0] first failing pivot (1-based) or 0; [1] solver error
     int* dFlags = nullptr;   // T+8 ints: ticket counters of the persistent solves
@@ -417,6 +418,7 @@ int lb_launch_kinv(lb_gp* h);
 int lb_launch_linv_levels(lb_gp* h, int want_tiles); // lml.cu: inverse of the diagonal blocks of `want_tiles` 128-tiles (power of two)
 int lb_launch_grad(lb_gp* h, int optimize_noise, double* dGrad);
 int lb_ensure_scratch(lb_gp* h, size_t bytes);
+int lb_query_int8_mode(); // query_i8.cu: int8 digit-product update of the panel query (LB_QUERY_INT8)
 int lb_tf32_prepare(lb_gp* h);
 int lb_launch_tf32_gemm_norm(cudaStream_t st, const void* dA, int64_t lda, const void* dB, int64_t ldb, int64_t M, int64_t N, int64_t K,
     int tri, float* dNorm2, float* dDout, int* dErr, int grid, int f16);

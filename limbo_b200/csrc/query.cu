@@ -825,15 +825,25 @@ LbOncePerDevice g_once;
 
 } // namespace panel
 
-// workspace in doubles behind dV (Np x Mp): Tbuf (SB * 128 x Mp) + norm partials (T x Mp)
+int lb_ldig_prepare(lb_gp* h);
+int lb_query_i8_vexp(const lb_gp* h);
+int64_t lb_query_int8_max_k();
+size_t lb_query_i8_vdig_bytes(int64_t Np, int64_t Mp);
+int lb_launch_vdig_split(cudaStream_t st, const double* dV, int64_t ld, int64_t Mp, int64_t r0, int64_t nr, int64_t c0, int64_t nc, int ev,
+    int8_t* dVdig);
+int lb_launch_panel_update_i8(const lb_gp* h, cudaStream_t st, const double* dV, const int8_t* dVdig, int64_t Mp, double* dT, int64_t ldt,
+    int s0, int nrows, int ct0, int n64, int ev, int* dErr);
+
+// workspace in doubles behind dV (Np x Mp): Tbuf (SB * 128 x Mp) + norm partials (T x Mp) [+ int8 digit planes of V (7 x Np x Mp bytes)]
 size_t lb_query_panel_scratch_doubles(const lb_gp* h, int64_t Mp)
 {
     const int64_t T = h->Np / LB_TILE;
-    return (size_t)(h->Np * Mp + (int64_t)panel::SB * LB_TILE * Mp + T * Mp);
+    const size_t vdig = lb_query_int8_mode() ? (lb_query_i8_vdig_bytes(h->Np, Mp) + 7) / 8 : 0;
+    return (size_t)(h->Np * Mp + (int64_t)panel::SB * LB_TILE * Mp + T * Mp) + vdig;
 }
 
 int lb_launch_query_panel(lb_gp* h, cudaStream_t st, int64_t M, const double* dQs, int64_t Mp, double* dWork, double* dMu, double* dS2,
-    long long* launches)
+    int* dErr, long long* launches)
 {
     using namespace panel;
     using CW = lbg::CfgWide;
@@ -851,6 +861,14 @@ int lb_launch_query_panel(lb_gp* h, cudaStream_t st, int64_t M, const double* dQ
     double* dNorm = dT + ldt * Mp;
     int rc = lb_launch_linv_levels(h, SB); // inverse of the 16-tile diagonal blocks (kept until the next fit)
     if (rc) return rc;
+    // int8 digit-product update (query_i8.cu) for the super-blocks with a K range inside its exactness bound
+    const bool i8 = lb_query_int8_mode() != 0;
+    int8_t* dVdig = i8 ? reinterpret_cast<int8_t*>(dNorm + (int64_t)T * Mp) : nullptr;
+    const int ev = i8 ? lb_query_i8_vexp(h) : 0;
+    if (i8) {
+        LbProfScope ps(h, st, LB_PC_QSTEP);
+        if ((rc = lb_ldig_prepare(h))) return rc; // digit planes of L (kept until the next fit)
+    }
     dim3 grid((unsigned)T, (unsigned)(Mp / LB_TILE));
     {
         LbProfScope ps(h, st, LB_PC_KSTAR);
@@ -926,18 +944,28 @@ int lb_launch_query_panel(lb_gp* h, cudaStream_t st, int64_t M, const double* dQ
         }
         for (int s0 = 0; s0 < T; s0 += SB) {
             const int nrows = (T - s0 < SB) ? (T - s0) : SB;
+            const bool upd_i8 = i8 && s0 > 0 && (int64_t)s0 * LB_TILE <= lb_query_int8_max_k();
             for (int g = 0; g < ngroups; ++g) {
                 const int c0 = gbeg[g] * wmul, nc = (gbeg[g + 1] - gbeg[g]) * wmul;
                 if (nc <= 0) continue;
-                if (dual) {
+                if (upd_i8) {
+                    const int n64 = (gbeg[g + 1] - gbeg[g]) * 2;
+                    if ((rc = lb_launch_panel_update_i8(h, sts[g], dV, dVdig, Mp, dT, ldt, s0, nrows, gbeg[g] * 2, n64, ev, dErr))) return rc;
+                }
+                else if (dual)
                     panel_update_kernel<CD, false><<<nrows * nc, CD::THREADS, CD::PIPE_BYTES, sts[g]>>>(h->dL, ld, dV, dT, ldt, s0, nrows, c0, 0, 1);
-                    panel_solve_kernel<CD, false><<<nrows * nc, CD::THREADS, CD::PIPE_BYTES, sts[g]>>>(h->dLinv, ld, dT, ldt, dV, s0, nrows, dNorm, Mp, c0, 0, 1);
-                }
-                else {
+                else
                     panel_update_kernel<CW, false><<<nrows * nc, CW::THREADS, CW::PIPE_BYTES, sts[g]>>>(h->dL, ld, dV, dT, ldt, s0, nrows, c0, 0, 1);
+                if (dual)
+                    panel_solve_kernel<CD, false><<<nrows * nc, CD::THREADS, CD::PIPE_BYTES, sts[g]>>>(h->dLinv, ld, dT, ldt, dV, s0, nrows, dNorm, Mp, c0, 0, 1);
+                else
                     panel_solve_kernel<CW, false><<<nrows * nc, CW::THREADS, CW::PIPE_BYTES, sts[g]>>>(h->dLinv, ld, dT, ldt, dV, s0, nrows, dNorm, Mp, c0, 0, 1);
-                }
                 if (launches) *launches += 2;
+                if (i8 && s0 + nrows < T) { // the solved rows feed the updates of the later super-blocks
+                    if ((rc = lb_launch_vdig_split(sts[g], dV, ld, Mp, (int64_t)s0 * LB_TILE, (int64_t)nrows * LB_TILE, (int64_t)gbeg[g] * LB_TILE,
+                             (int64_t)(gbeg[g + 1] - gbeg[g]) * LB_TILE, ev, dVdig))) return rc;
+                    if (launches) ++*launches;
+                }
             }
         }
         for (int g = 1; g < ngroups; ++g) { // join (ev[1..3]; the fit's uses of these events are complete: same stream order)

@@ -21,14 +21,15 @@
 // Around them: kstar_t32_kernel (K*^T chunk from fp64 kernel evaluations with the squared distances on the fp64 tensor pipe,
 // mean and rounding-bias partials fused), mu_reduce_kernel, sigma2_t32_kernel (clamp / noise of gp.hpp:623,166 and the
 // rounding-bias correction), linv_to_rowmajor_kernel (+ absmax / colnorm2 for the fp16 scale and the bias weights).
-#include "common.cuh"
-#include <cuda.h>
+#include "tcgen05.cuh"
 #include <cuda_fp16.h>
 #include <cmath>
 #include <type_traits>
 #include <cstdlib>
 
 namespace tf32q {
+
+using namespace lbtc;
 
 constexpr int BM = 128;       // candidates per tile (UMMA M)
 constexpr int BN = 256;       // outputs (rows of L^-1) per tile (UMMA N)
@@ -41,72 +42,6 @@ constexpr int B_BYTES = BN * 128;  // 32 KB
 constexpr int STAGE_BYTES = A_BYTES + B_BYTES;
 constexpr int THREADS = 192;
 constexpr size_t SMEM_BYTES = (size_t)STAGES * STAGE_BYTES + 1024 /*align*/ + 256 /*barriers*/;
-constexpr long long SPIN_LIMIT = 1LL << 24;
-
-__device__ __forceinline__ void mbar_init(uint64_t* b, uint32_t n)
-{
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(lb_smem_u32(b)), "r"(n));
-}
-__device__ __forceinline__ void mbar_expect_tx(uint64_t* b, uint32_t bytes)
-{
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(lb_smem_u32(b)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint64_t* b)
-{
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(lb_smem_u32(b)) : "memory");
-}
-__device__ __forceinline__ bool mbar_try(uint64_t* b, uint32_t parity)
-{
-    uint32_t ok;
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(ok)
-        : "r"(lb_smem_u32(b)), "r"(parity)
-        : "memory");
-    return ok != 0;
-}
-// bounded wait: returns false (and raises *err) instead of spinning forever
-// The error flag (global memory) is polled only every 1024 attempts: a volatile load per spin from six spinning warps
-// would saturate the SM's load/store path (and starve any kernel sharing the SM).
-__device__ __forceinline__ bool mbar_wait(uint64_t* b, uint32_t parity, int* err)
-{
-    long long spins = 0;
-    while (!mbar_try(b, parity)) {
-        if ((++spins & 1023) == 0 && (spins > SPIN_LIMIT || *(volatile int*)err)) {
-            atomicExch(err, 1);
-            return false;
-        }
-    }
-    return true;
-}
-// Long waits of a whole warp (epilogue waiting for ~100 us of MMAs): one lane polls with a back-off, the other 31 lanes
-// sleep at the warp barrier instead of issuing try_wait / branch instructions.
-__device__ __forceinline__ bool mbar_wait_warp(uint64_t* b, uint32_t parity, int* err)
-{
-    int ok = 1;
-    if ((threadIdx.x & 31) == 0) {
-        long long spins = 0;
-        while (!mbar_try(b, parity)) {
-            __nanosleep(128);
-            if ((++spins & 255) == 0 && (spins > (SPIN_LIMIT >> 4) || *(volatile int*)err)) {
-                atomicExch(err, 1);
-                ok = 0;
-                break;
-            }
-        }
-    }
-    ok = __shfl_sync(0xffffffffu, ok, 0);
-    return ok != 0;
-}
-__device__ __forceinline__ void tma_load_2d(void* dst, const CUtensorMap* map, int c0, int c1, uint64_t* bar)
-{
-    asm volatile("cp.async.bulk.tensor.2d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];" ::"r"(
-                     lb_smem_u32(dst)),
-                 "l"(map), "r"(c0), "r"(c1), "r"(lb_smem_u32(bar))
-                 : "memory");
-}
 // K-major, SWIZZLE_128B shared-memory matrix descriptor (cute::UMMA::SmemDescriptor, mma_sm100_desc.hpp):
 //   [0,14) start address >> 4 | [16,30) leading byte offset >> 4 (unused for swizzled K-major: 1) |
 //   [32,46) stride byte offset >> 4 (8 rows x 128 B = 1024 B -> 64) | [46,48) version = 1 | [61,64) layout = 2 (SWIZZLE_128B)
@@ -141,23 +76,6 @@ __device__ __forceinline__ void umma(uint32_t d_tmem, uint64_t adesc, uint64_t b
             ::"r"(d_tmem), "l"(adesc), "l"(bdesc), "r"(idesc<false>()), "r"(accumulate)
             : "memory");
 }
-__device__ __forceinline__ void umma_commit(uint64_t* bar)
-{
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(lb_smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&v)[32])
-{
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x32.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
-        "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];"
-        : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]), "=r"(v[9]),
-          "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15]), "=r"(v[16]), "=r"(v[17]), "=r"(v[18]),
-          "=r"(v[19]), "=r"(v[20]), "=r"(v[21]), "=r"(v[22]), "=r"(v[23]), "=r"(v[24]), "=r"(v[25]), "=r"(v[26]), "=r"(v[27]),
-          "=r"(v[28]), "=r"(v[29]), "=r"(v[30]), "=r"(v[31])
-        : "r"(taddr)
-        : "memory");
-}
-
 // D[c, n] = sum_k A[c, k] B[n, k]; tri != 0: k only up to the end of the n-tile (B lower triangular).
 // norm2[c] += sum_n D[c, n]^2 ; Dout (optional, row-major M x N) receives D for validation.
 template <bool F16>
@@ -774,21 +692,6 @@ pair_split_gemm_norm_kernel(const __grid_constant__ CUtensorMap mapAh, const __g
         asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
         asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512) : "memory");
     }
-}
-
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-    const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-static EncodeTiledFn get_encode()
-{
-    static EncodeTiledFn fn = nullptr;
-    if (!fn) {
-        void* p = nullptr;
-        cudaDriverEntryPointQueryResult qres;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &qres) == cudaSuccess && qres == cudaDriverEntryPointSuccess)
-            fn = (EncodeTiledFn)p;
-    }
-    return fn;
 }
 
 // row-major (rows x K) fp32 matrix, boxes of 32 k x box_rows rows, 128-byte swizzle, tf32 rounding on load
